@@ -2,7 +2,7 @@
 """bench.py — learner transitions/s for the Ape-X hot path (sample + gather +
 target + priority update, inside a full learner step) on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md §8d C2): Ape-X DQN, 2^20-slot
 device-resident sum-tree per GPU, synthetic (4,84,84) uint8 frame stacks (59.2 GB
@@ -49,7 +49,7 @@ ALG_BYTES_PER_TRANSITION_GATHER = 2 * 28224 + 4 + 4 + 1   # SURVEY.md §8d: 56 4
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 1000 for apex, 40 for r2d2 / impala)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="apex", choices=["apex", "r2d2", "impala"],
@@ -68,7 +68,6 @@ def parse():
     ap.add_argument("--unfused-tail", action="store_true", help="dueling tail as separate PyTorch ops instead of csrc/dueling.cu")
     ap.add_argument("--cublas-dense", action="store_true", help="dense heads as cuBLAS fp32 GEMMs instead of the 3xTF32 tcgen05 kernel (csrc/gemm.cu)")
     ap.add_argument("--torch-optim", action="store_true", help="torch.optim.RMSprop instead of the fused kernel")
-    ap.add_argument("--no-cudnn-benchmark", action="store_true", help="leave cuDNN's algorithm choice to its heuristics")
     ap.add_argument("--blaslt", action="store_true", help="route fp32 GEMMs through cuBLASLt")
     ap.add_argument("--tf32-matmul", action="store_true",
                     help="INFORMATIONAL ONLY: let the dense heads use TF32 like cuDNN's convolutions already do "
@@ -80,7 +79,52 @@ def parse():
                          "the line it prints is NOT a bench result")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=48)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 1000 if args.workload == "apex" else 40
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl b200)")
+    return args
+
+
+def reproducible_cudnn():
+    """cuDNN picks the conv_2 / conv_3 algorithms with its heuristics (mode B) among the deterministic ones instead
+    of timing candidates (cudnn.benchmark).  Timing can pick differently from run to run; one step that rounds
+    differently changes the priorities and with them the minibatches of every later step.  This way the same
+    arguments compute the same outputs on every run.  Must run before the process's first convolution."""
+    import torch
+    os.environ.setdefault("TORCH_CUDNN_USE_HEURISTIC_MODE_B", "1")
+    torch.backends.cudnn.benchmark = False
+    torch.backends.cudnn.deterministic = True
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outdir, outputs, rank=0):
+    """Write a step's returned tensors as `outdir/<name>.npy` so that two builds can be compared output for output:
+    fp32 (and narrower) floats as float32, everything else (int64 indices, fp64) as float64.  Past
+    DUMP_LIMIT_BYTES in all, every array is cut to the same fixed, seeded sample of its elements.  Rank r > 0
+    of a multi-GPU run writes `<name>_rank<r>.npy`."""
+    import numpy as np
+    import torch
+
+    arrays = {}
+    for name, t in outputs.items():
+        t = torch.as_tensor(t).detach()
+        small_float = t.is_floating_point() and t.element_size() <= 4
+        arrays[name] = t.to("cpu", torch.float32 if small_float else torch.float64).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES:
+            keep = max(1, a.size * DUMP_LIMIT_BYTES // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(outdir, name + (f"_rank{rank}" if rank else "") + ".npy"), a)
 
 
 # --------------------------------------------------------------------------- #
@@ -295,9 +339,9 @@ def secondary_workload(args):
         raise SystemExit("bench.py needs a CUDA device (the product path has no CPU fallback)")
     dev = torch.device("cuda", 0)
     torch.cuda.set_device(dev)
-    torch.backends.cudnn.benchmark = not args.no_cudnn_benchmark
+    reproducible_cudnn()
     lib = _lib.load()
-    steps = args.steps if args.steps != 1000 else 40
+    steps = args.steps
     warm = max(3, min(args.warmup, 5))
     g = torch.Generator(device=dev); g.manual_seed(0xB200 + 7)
     peaks = {}
@@ -396,6 +440,8 @@ def secondary_workload(args):
     ms, out = timed_region(steps)
     launches = lib.b2rl_launch_count() - c0
     clock_info = clocks.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     value = units * (T if args.workload == "r2d2" else T) * steps / (ms / 1e3)
 
     # ---- dominant hand-written kernel alone: fused in-place gather + conv_1 over one step's frames ----
@@ -506,7 +552,7 @@ def main():
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     # library knobs for the PyTorch remainder of the network (no precision change: fp32 matmul, TF32 conv)
-    torch.backends.cudnn.benchmark = not args.no_cudnn_benchmark
+    reproducible_cudnn()
     if args.cudnn_conv1_wgrad:
         from distributed_rl_b200.apex import _Conv1Gathered
         _Conv1Gathered.fused_wgrad = False
@@ -523,7 +569,8 @@ def main():
     N, B = 1 << args.log2n, args.batch
     cfg = ApexConfig(BATCHSIZE=B, REPLAY_MEMORY_LEN=N, BUFFER_SIZE=0, LEARNER_DEVICE=str(dev),
                      CHANNELS_LAST=not args.nchw, FUSED_CONV1=not args.unfused_conv1,
-                     FUSED_OPTIM=not args.torch_optim, DENSE_3XTF32=not args.cublas_dense, FUSED_DUELING_TAIL=not args.unfused_tail, PARALLEL_FORWARDS=not args.serial_forwards, DEFERRED_WGRAD=not args.inline_wgrad)
+                     FUSED_OPTIM=not args.torch_optim, DENSE_3XTF32=not args.cublas_dense, FUSED_DUELING_TAIL=not args.unfused_tail, PARALLEL_FORWARDS=not args.serial_forwards, DEFERRED_WGRAD=not args.inline_wgrad,
+                     CUDNN_BENCHMARK=False)
     torch.manual_seed(0)
     learner = Learner(cfg, connect=None, start_replay=False)
     if world > 1:   # identical initial weights on every rank
@@ -570,6 +617,8 @@ def main():
     clock_info = clocks.stop() if clocks else None
     value = B * world * args.steps / (ms / 1e3)
     scal = out["scalars"].tolist()
+    if args.dump_outputs:     # before anything else replays the step graph, whose outputs `out` holds
+        dump_outputs(args.dump_outputs, out, rank)
 
     if args.quick:
         if rank == 0:

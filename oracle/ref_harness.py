@@ -3,8 +3,8 @@
 Imports seungju-k1m/Distributed_RL from /root/reference (read-only, never copied)
 so that `tests/golden/make_golden.py` can execute the reference's own functions
 and record their outputs as golden vectors.  /root/reference does not exist on
-the GPU box, so nothing under tests/ -m gpu, bench.py or smoke() may import
-this module; only the golden generator and the `needs_reference` CPU tests do.
+GPU machines, so nothing under tests/ -m gpu, bench.py or smoke() may use
+this module to load it; only the golden generator does.
 
 What has to be shimmed for the reference to import under python 3.12 /
 numpy 2.3 / torch 2.11 (SURVEY.md §8c):

@@ -15,18 +15,6 @@ GOLDEN = os.path.join(REPO, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "needs_reference: executes /root/reference (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    from oracle.ref_harness import reference_available
-
-    if reference_available():
-        return
-    skip = pytest.mark.skip(reason="/root/reference not present on this machine")
-    for it in items:
-        if "needs_reference" in it.keywords:
-            it.add_marker(skip)
 
 
 @pytest.fixture(autouse=True)

@@ -16,6 +16,7 @@ Groups
   apex    APE_X/Learner.py Learner.train   (Q-values captured by wrapping forward)
   r2d2    R2D2/Learner.py Learner.train    (MEM=40, SURVEY §8a-note 1)
   impala  IMPALA/Learner.py Learner.train  (V-trace internals captured at calLoss)
+  dropin  run_learner.py's Learner binding + baseline/baseAgent.py Q-values on seeded weights
 """
 from __future__ import annotations
 
@@ -451,8 +452,34 @@ def gen_impala_e2e():
     print("impala_e2e.npz:", len(out), "arrays")
 
 
+def gen_dropin():
+    """What the drop-in tests compare with: the Learner class the reference's run_learner.py binds under the Ape-X
+    cfg, and the reference baseAgent's parameter names, shapes and Q-values on seeded weights and a seeded input."""
+    import runpy
+    import numpy as np
+    import torch
+    from oracle import ref_harness as H
+
+    H.enter_reference("ape_x.json")
+    L = runpy.run_path(os.path.join(H.REFERENCE_ROOT, "run_learner.py"), run_name="not_main")["Learner"]
+    import configuration as C  # type: ignore
+    from baseline.baseAgent import baseAgent  # type: ignore
+
+    net = baseAgent(C.MODEL)
+    names = _load_seeded(net, 606)
+    x = np.random.default_rng(0xB200 + 66).random((5, 4, 84, 84), dtype=np.float32)
+    with torch.no_grad():
+        q = net.forward([torch.from_numpy(x)])[0].numpy()
+    out = {"run_learner_alg": np.array(C.ALG), "run_learner_class": np.array(f"{L.__module__}.{L.__qualname__}"),
+           "agent_names": np.array(names),
+           "agent_shapes": np.array(["x".join(map(str, v.shape)) for v in net.state_dict().values()]),
+           "agent_q": q}
+    np.savez_compressed(os.path.join(HERE, "dropin.npz"), **out)
+    print("dropin.npz:", len(out), "arrays")
+
+
 GROUPS = {"tree": gen_tree, "apex": gen_apex, "r2d2": gen_r2d2, "impala": gen_impala, "apex_e2e": gen_apex_e2e,
-          "r2d2_e2e": gen_r2d2_e2e, "impala_e2e": gen_impala_e2e}
+          "r2d2_e2e": gen_r2d2_e2e, "impala_e2e": gen_impala_e2e, "dropin": gen_dropin}
 
 if __name__ == "__main__":
     want = sys.argv[1:] or list(GROUPS)

@@ -40,12 +40,15 @@ def _worker(rank, world, port, q):
     b2 = D.FlatGradBucket(lin2.parameters())
     b2.enable_overlap([lin2[1].weight])          # the last layer's gradient is ready first
     lin2(x).sum().backward()
-    local2 = [p.grad.clone() for p in lin2.parameters()]
     b2.finish()
+    # the early all-reduce runs asynchronously in place, so this rank's own gradients come from a replica
+    ref2 = torch.nn.Sequential(torch.nn.Linear(4, 3, bias=False), torch.nn.Linear(3, 2, bias=False))
+    ref2.load_state_dict(lin2.state_dict())
+    ref2(x).sum().backward()
     ok = True
-    for p, l in zip(lin2.parameters(), local2):
-        g = [torch.zeros_like(l) for _ in range(world)]
-        dist.all_gather(g, l)
+    for p, r in zip(lin2.parameters(), ref2.parameters()):
+        g = [torch.zeros_like(r.grad) for _ in range(world)]
+        dist.all_gather(g, r.grad)
         ok = ok and bool(torch.allclose(p.grad, sum(g) / world))
     out["overlap_ok"] = ok
     # 1c. early gradients that bypass AccumulateGrad (linear.WeightGradSink): the sink's on_ready callback

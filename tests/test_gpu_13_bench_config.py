@@ -1,6 +1,6 @@
 """Parity AT THE BENCHMARKED CONFIGURATION (bench.py, BASELINE.json configs[1]): Ape-X, 2^20 slots, batch 512, the whole
-step replayed as a CUDA graph, PyTorch's default library precision (TF32 convolutions, cuDNN autotune) — what the
-driver's bench line is measured on, not a reduced stand-in."""
+step replayed as a CUDA graph, PyTorch's default library precision (TF32 convolutions) with cuDNN's heuristic, deterministic
+algorithm choice — what bench.py's line is measured on, not a reduced stand-in."""
 import numpy as np
 import pytest
 
@@ -24,11 +24,11 @@ def test_graph_replays_at_bench_config_match_the_oracle_step_by_step():
     if free < 70 << 30:
         pytest.skip("needs ~62 GB of free HBM (2^20 Ape-X slots)")
     from distributed_rl_b200 import apex, replay as R
-    torch.backends.cudnn.benchmark = True              # the bench's library knobs (bench.py main)
-    torch.backends.cudnn.deterministic = False
+    torch.backends.cudnn.benchmark = False             # the bench's library knobs (bench.py reproducible_cudnn)
+    torch.backends.cudnn.deterministic = True
     torch.backends.cudnn.allow_tf32 = True
     N = 1 << LOG2N
-    cfg = apex.ApexConfig(BATCHSIZE=B, REPLAY_MEMORY_LEN=N, BUFFER_SIZE=0, LEARNER_DEVICE="cuda:0")
+    cfg = apex.ApexConfig(BATCHSIZE=B, REPLAY_MEMORY_LEN=N, BUFFER_SIZE=0, LEARNER_DEVICE="cuda:0", CUDNN_BENCHMARK=False)
     torch.manual_seed(0)
     L = apex.Learner(cfg, connect=None, start_replay=False)
     st = L.memory.store

@@ -1,5 +1,5 @@
 import os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from distributed_rl_b200 import replay as R
 N = 1 << 20
